@@ -2,7 +2,7 @@
 """bench.py -- N-pair fwd+bwd samples/sec (BASELINE.json metric: B=8192, D=512 on 1/2/4/8 B200).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config HL|C2|C3|C4|C5]
-                  [--precision fp16x2|bf16x3|bf16] [--mining config|usage|rand|relative]
+                  [--precision fp16x2|bf16x3|bf16] [--mining config|usage|rand|relative] [--dump-outputs DIR]
 
 One "step" = Forward_gpu + Backward_gpu of the NPairMultiClassLoss layer (reference npair_multi_class_loss.cu:207-402, :420-499)
 over one batch of synthetic L2-normalised embeddings (B/2 classes x 2 images, SURVEY 8d seeds), the global batch sharded by anchor
@@ -46,6 +46,7 @@ import time  # noqa: E402
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the source tree as it found it (it may be read-only)
 
 import numpy as np  # noqa: E402
 
@@ -147,7 +148,6 @@ def metric_name(B, D):
 def oracle_sample(B, D, mining, x, lab, world_s, threads):
     """The oracle state for the bounded CPU sample: rank 0's block of a world_s-way anchor sharding, faithful sorts, fp32 accumulate."""
     from oracle import oracle_lib as o
-    o.build()
     Qs = B // world_s
     cfg = o.make_config(Qs, D, world=world_s, rank=0, accum_double=0, faithful_sorts=1, num_threads=threads, **mining)
     L = o.lib()
@@ -205,6 +205,39 @@ def run_reference(args, wl):
     emit(out)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, tops, grad, world, rank):
+    """Writes what the step call returned in the last timed step, as float32 .npy files under `path` (rank 0):
+      tops.npy  (world, 5)  loss, top1, top5, top10, feature_asum of every rank
+      dx.npy    (B, D)      the gradient of the whole batch, rank blocks in order
+    When dx would exceed the size cap, a fixed, seeded sample of its rows is written instead, as dx_sample.npy, with the row
+    indices in dx_sample_rows.npy (float64).  The inputs depend only on the arguments, so two builds run with the same
+    arguments can be compared file by file."""
+    import torch
+    import torch.distributed as dist
+    t = torch.tensor(tops, dtype=torch.float32, device=grad.device).reshape(1, 5)
+    if world > 1:
+        ts = [torch.empty_like(t) for _ in range(world)]
+        gs = [torch.empty_like(grad) for _ in range(world)]
+        dist.all_gather(ts, t)
+        dist.all_gather(gs, grad)
+        t, grad = torch.cat(ts), torch.cat(gs)
+    if rank != 0:
+        return
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "tops.npy"), t.cpu().numpy())
+    B, D = grad.shape
+    cap = DUMP_BYTES - (1 << 20)                         # the rest is room for tops.npy and the .npy headers
+    if B * D * 4 <= cap:
+        np.save(os.path.join(path, "dx.npy"), grad.cpu().numpy())
+        return
+    rows = np.sort(np.random.default_rng(20171225).choice(B, size=cap // (4 * D + 8), replace=False))
+    np.save(os.path.join(path, "dx_sample.npy"), grad[torch.from_numpy(rows).to(grad.device)].cpu().numpy())
+    np.save(os.path.join(path, "dx_sample_rows.npy"), rows.astype(np.float64))
+
+
 _REAL_STDOUT = None
 
 
@@ -241,7 +274,12 @@ def main():
     ap.add_argument("--no-flush", action="store_true", help="diagnostic: never flush the L2 between steps (sharded runs)")
     ap.add_argument("--cfg-flags", type=int, default=0, help="npair_config.flags (NPAIR_FLAG_*), e.g. 24 = exchange through NCCL instead of peer memory")
     ap.add_argument("--grad-chunk", type=int, default=0, help="npair_config.grad_chunk_cols (0 = library default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the tops and the gradient of the last timed step as DIR/<name>.npy (float32, "
+                         "at most 64 MB: a seeded sample of the rows of a larger gradient), to compare two builds output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU step (--impl ours)")
 
     from npairloss_b200 import synth
     wl = resolve_workload(args)
@@ -327,7 +365,7 @@ def main():
     flush_buf = torch.empty(2 * L2_BYTES, dtype=torch.uint8, device=dev) if need_flush else None
 
     def timed_steps(c, steps, fn=None):
-        """ms per step (this rank), kernel launches inside the region."""
+        """ms per step (this rank), kernel launches inside the region, the tops of the last step."""
         fn = fn or step_device
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier()
@@ -335,21 +373,21 @@ def main():
             e0.record(stream)
             l0 = capi.kernel_launches()
             for _ in range(steps):
-                fn(c)
+                t = fn(c)
             nl = capi.kernel_launches() - l0
             e1.record(stream)
             barrier()
-            return e0.elapsed_time(e1) / steps, nl
+            return e0.elapsed_time(e1) / steps, nl, t
         pairs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
         l0 = capi.kernel_launches()
         for ea, eb in pairs:
             flush_buf.fill_(1)                 # same stream as the step: ordered before it, evicts the whole L2
             ea.record(stream)
-            fn(c)
+            t = fn(c)
             eb.record(stream)
         nl = capi.kernel_launches() - l0
         barrier()
-        return float(sum(ea.elapsed_time(eb) for ea, eb in pairs)) / steps, nl
+        return float(sum(ea.elapsed_time(eb) for ea, eb in pairs)) / steps, nl, t
 
     def max_over_ranks(v):
         t = torch.tensor([v], dtype=torch.float64, device=dev)
@@ -365,7 +403,8 @@ def main():
         tops = step_device()
     barrier()
     n_before = len(sampler.rows)
-    ms_mine, launches_timed = timed_steps(ctx, args.steps)
+    ms_mine, launches_timed, tops_timed = timed_steps(ctx, args.steps)
+    grad_timed = d_g.clone() if args.dump_outputs else None      # later legs reuse d_g
     clocks = None
     if rank == 0:
         in_region = len(sampler.rows) - n_before
@@ -535,7 +574,7 @@ def main():
             c2 = make_ctx(m)
             for _ in range(3):
                 step_device(c2)
-            ms2, _ = timed_steps(c2, 20)
+            ms2 = timed_steps(c2, args.steps)[0]
             ms2 = max_over_ranks(ms2)
             ph2 = profile_phases(c2, 5)
             c2.close()
@@ -597,7 +636,6 @@ def main():
         dist.all_gather(ts_all, torch.tensor(ts, device=dev, dtype=torch.float32))
         if rank == 0:
             from oracle import oracle_lib as o
-            o.build()
             ocfg = o.make_config(Qs, Ds, world=world, faithful_sorts=0, **synth.USAGE_MINING)
             tops_o, dx_o = o.step_world(xs, ls, ocfg, 0.7, S_inject_all=torch.cat(S_all).cpu().numpy())
             dxg = torch.cat(g_all).cpu().numpy()
@@ -648,6 +686,8 @@ def main():
                "gpu_launches": launches_timed,
                "tops": {"loss": tops[0], "top1": tops[1], "top5": tops[2], "top10": tops[3], "feature_asum": tops[4]}}
         emit(out)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, tops_timed, grad_timed, world, rank)
     ctx.close()
     if world > 1:
         dist.destroy_process_group()

@@ -58,9 +58,10 @@ def test_parse_reference_usage_block():
     assert (p["ap_region"], p["ap_method"], p["an_region"], p["an_method"]) == (0, 3, 1, 0)
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/usage/def.prototxt"), reason="reference tree only exists in the build container")
 def test_parse_reference_prototxt_file_unchanged():
-    txt = open("/root/reference/usage/def.prototxt", encoding="utf-8", errors="replace").read()
+    """usage/def.prototxt of the reference, stored byte for byte as tests/golden/usage_def.prototxt."""
+    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "usage_def.prototxt")
+    txt = open(path, encoding="utf-8", errors="replace").read()
     p = caffe_layer.parse_only(txt)
     assert p["num_tops"] == 5 and p["n_loss_weights"] == 5
     assert (p["ap_region"], p["ap_method"], p["an_region"], p["an_method"]) == (0, 3, 1, 0)
